@@ -62,6 +62,9 @@ def parse():
                     help="N>1: template shard layout (interleaved: rank r takes templates r, r+N, ...: even candidate load)")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run result check against the oracle")
     ap.add_argument("--seed", type=int, default=1234)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the match list of the last timed step (what lm_finish hands a caller) "
+                         "as DIR/matches_<field>.npy, to compare two builds on the same inputs")
     return ap.parse_args()
 
 
@@ -200,6 +203,21 @@ def oracle_expected(args, packed, quantized, world):
     return oracle.match(quantized, T_PYR, packed, args.threshold, n_threads=min(threads, 64))
 
 
+DUMP_BYTES = 60 * 10 ** 6   # rows of a dump; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, matches):
+    """One .npy per field of a match list, one row per match: similarity float32, the integer fields float64 (exact).  A
+    list of more than DUMP_BYTES is cut to a fixed, seeded sample of its rows, kept in order."""
+    os.makedirs(out_dir, exist_ok=True)
+    dtypes = {f: np.float32 if f == "similarity" else np.float64 for f in matches.dtype.names}
+    row_bytes = sum(np.dtype(t).itemsize for t in dtypes.values())
+    if len(matches) * row_bytes > DUMP_BYTES:
+        matches = matches[np.sort(np.random.default_rng(0).choice(len(matches), DUMP_BYTES // row_bytes, replace=False))]
+    for f, t in dtypes.items():
+        np.save(os.path.join(out_dir, "matches_%s.npy" % f), matches[f].astype(t))
+
+
 def same_matches(got, want):
     if len(got) != len(want):
         return False
@@ -228,9 +246,8 @@ def real_data_arm(lib, torch, local):
     (tests/golden/expected_allScales_full.npz).  One frame repeated, i.e. L2-resident inputs: a candidate-load check of
     the kernels on real data, not a second headline."""
     g = os.path.join(ROOT, "tests", "golden")
-    b = np.load(os.path.join(g, "bank_allScales_full.npz"))
-    packed = dict(class_begin=b["class_begin"], tmeta=b["tmeta"].astype(np.int32), feats=b["feats"].astype(np.int32))
-    T = b["T"].tolist()
+    from oracle import golden
+    packed, T = golden.allscales_full_bank()
     fr = np.load(os.path.join(g, "frames_case1.npz"))
     q = [[np.ascontiguousarray(fr["full_l%d_m%d" % (l, m)]) for m in range(2)] for l in range(2)]
     exp = np.load(os.path.join(g, "expected_allScales_full.npz"))
@@ -294,12 +311,12 @@ def threshold_sweep(lib, torch, local, args, packed, ring, rows, cols):
 def pose_pipeline(lib, local):
     """BASELINE.json config 3 as ONE figure: raw RGB-D frame -> match -> greedy NMS top-3 on the device -> poseRefine of the
     three hypotheses (max 10 ICP iterations) in one batched call.  Inputs: the frame, bank and render of the recorded
-    driver run (tests/golden/driver_trace.npz, bank_allScales_full.npz).  Pose error against the ICP oracle with the same
-    iteration cap (PARITY UNPINNED: the reference's ICP arithmetic is Open3D's, see oracle/icp_oracle.py)."""
+    driver run (tests/golden/driver_trace.npz, bank_allScales_full_{a,b}.npz).  Pose error against the ICP oracle with the
+    same iteration cap (PARITY UNPINNED: the reference's ICP arithmetic is Open3D's, see oracle/icp_oracle.py)."""
     g = os.path.join(ROOT, "tests", "golden")
     tr = np.load(os.path.join(g, "driver_trace.npz"))
-    b = np.load(os.path.join(g, "bank_allScales_full.npz"))
-    packed = dict(class_begin=b["class_begin"], tmeta=b["tmeta"].astype(np.int32), feats=b["feats"].astype(np.int32))
+    from oracle import golden
+    packed, _ = golden.allscales_full_bank()
     nat = lib.NativeDetector(tr["T"].tolist(), device=local)
     nat.load_bank(packed, 4)
     nat.set_boxes(np.full((int(packed["class_begin"][-1]), 2), 70, np.int32))  # the driver's info files: 70 x 70 boxes
@@ -497,6 +514,24 @@ def main():
         launches = int(lt.item())
     fps = args.steps / (ms / 1e3)
 
+    def finished(n_, host):
+        """The match list of the last frame `n_` completed, as lm_finish hands it to a caller.  host: every rank's result
+        block after the NCCL all-gather, or None when the records sit in the handle's own block."""
+        if host is not None:
+            blocks = host.numpy().reshape(world, blk_bytes)
+            rec = np.concatenate([blocks[r, 16:16 + 16 * int(blocks[r, :4].view(np.int32)[0])].view(lib.RECORD_DTYPE)
+                                  for r in range(world)])
+        else:
+            rec = n_.fetch_records()
+        return n_.finish(rec)
+
+    if args.dump_outputs:
+        if rank == 0:
+            last = args.warmup + args.steps - 1
+            dump_outputs(args.dump_outputs, finished(nats[last % len(nats)] if (fused or world == 1) else nat,
+                                                     gathered.cpu() if (world > 1 and not fused) else None))
+        barrier()
+
     # ---- result check: the frames at both ends of the timed region, through every lane (same calls as the timed loop:
     # bind -> enqueue -> complete), against the oracle's list.  A mismatch fails the run.
     parity = {"checked": False, "ok": None, "frames": 0}
@@ -514,13 +549,7 @@ def main():
                     host = gathered.to("cpu", non_blocking=False)
             for k_, n_ in enumerate(nats if (fused or world == 1) else nats[:1]):
                 n_.complete()
-                if world > 1 and not fused:
-                    blocks = host.numpy().reshape(world, blk_bytes)
-                    rec = np.concatenate([blocks[r, 16:16 + 16 * int(blocks[r, :4].view(np.int32)[0])].view(lib.RECORD_DTYPE)
-                                          for r in range(world)])
-                else:
-                    rec = n_.fetch_records()
-                got = n_.finish(rec)
+                got = finished(n_, host if (world > 1 and not fused) else None)
                 good = same_matches(got, want)
                 if not good:
                     sys.stderr.write("PARITY MISMATCH rank %d lane %d frame %d: got %d matches, oracle %d\n" % (rank, k_, fi, len(got), len(want)))

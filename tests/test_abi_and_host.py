@@ -96,21 +96,18 @@ def test_bank_yaml_round_trip(tmp_path, synth):
         bk.TemplateBank().read_class(fmt % "03_template", 3)  # pyramid_levels mismatch, LL.cpp:2052
 
 
-REF_CASE = "/root/reference/linemodLevelup/test/case1/"
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_CASE), reason="/root/reference not mounted")
-def test_reads_the_reference_fixture_banks():
+def test_reads_the_reference_fixture_banks(tmp_path):
+    from test_bank_packed import write_reference_yaml
     bk = importlib.import_module("6dpose_b200.bank")
     b = bk.TemplateBank()
-    b.read_class(REF_CASE + "127/06_template.yaml", 2)
+    b.read_class(write_reference_yaml("127", str(tmp_path / "127.yaml")), 2)
     tps = b.classes["06_template"]
     assert len(tps) == 89 and len(tps[0]) == 4
     assert tps[0][0].features.shape == (127, 3) and tps[0][2].features.shape == (63, 3)
     assert (tps[0][0].width, tps[0][0].height) == (37, 72)
     assert tps[0][0].features[0].tolist() == [3, 12, 0]
     old = bk.TemplateBank()
-    old.read_class(REF_CASE + "writeClasses/06_template.yaml", 2)   # older dialect with an extra depth: key
+    old.read_class(os.path.join(ROOT, "tests", "golden", "writeClasses_06_template.yaml.gz"), 2)   # older dialect, float depth: key
     assert old.num_templates() == 1
 
 

@@ -1,5 +1,6 @@
 """Packed bank files (SURVEY.md section 8f-4): lossless against the YAML dialect of the reference
 (LL.cpp:2093-2146), integrity-checked, and usable through Detector.readClasses / writeClasses."""
+import hashlib
 import importlib
 import os
 import time
@@ -19,6 +20,32 @@ def bank_from_golden(name, class_id="06_template"):
     tm = g["tmeta"].copy()
     b.classes[class_id] = bk.PackedPyramids(tm, g["feats"], tm.shape[1] // 2)
     return b
+
+
+def write_reference_yaml(name, path):
+    """Writes the reference's bank file test/case1/<name>/06_template.yaml (name: 127 or allScales) byte for byte from the
+    golden bank, adding the per-template `depth:` lines the bank arrays do not hold; checked against the file's SHA-256
+    (tests/golden/make_golden.py)."""
+    g = np.load(os.path.join(HERE, "golden", "reference_yaml.npz"))
+    if name == "allScales":
+        from oracle import golden
+        packed, _ = golden.allscales_full_bank()
+        b = bk.TemplateBank()
+        b.classes["06_template"] = bk.PackedPyramids(packed["tmeta"], packed["feats"], 2)
+    else:
+        b = bank_from_golden("bank_%s.npz" % name)
+    b.write_class("06_template", path, 2)
+    if name + "_depth" in g.files:
+        depth = iter(g[name + "_depth"].ravel().tolist())
+        lines = []
+        for ln in open(path).read().split("\n"):
+            lines.append(ln)
+            if ln.startswith("            pyramid_level: "):
+                lines.append("            depth: %d" % next(depth))
+        with open(path, "w") as fh:
+            fh.write("\n".join(lines))
+    assert hashlib.sha256(open(path, "rb").read()).hexdigest() == str(g[name + "_sha256"]), name
+    return path
 
 
 def same_pack(a, b):
@@ -56,12 +83,9 @@ def test_reference_fixture_bank_survives_packing(tmp_path):
     assert same_pack(r.pack(["06_template"], 4), want)
 
 
-REF_BANK = "/root/reference/linemodLevelup/test/case1/allScales/06_template.yaml"
-
-
-@pytest.mark.skipif(not os.path.exists(REF_BANK), reason="/root/reference not mounted")
 def test_full_reference_bank_yaml_vs_packed(tmp_path):
     """The reference's own 2989-template YAML: parse, pack, reload -- identical, much smaller and faster."""
+    REF_BANK = write_reference_yaml("allScales", str(tmp_path / "allScales.yaml"))
     t0 = time.perf_counter()
     y = bk.TemplateBank()
     y.read_class(REF_BANK, 2)

@@ -1,13 +1,12 @@
-"""The shared cv2 quantization front-end (6dpose_b200/frontend.py): tables against the reference
-file when mounted, filters against naive per-pixel restatements."""
+"""The shared cv2 quantization front-end (6dpose_b200/frontend.py): tables against the reference's
+(tests/golden/reference_tables.npz), filters against naive per-pixel restatements."""
 import importlib
 import os
-import re
 
 import numpy as np
 import pytest
 
-REF_LUT = "/root/reference/linemodLevelup/normal_lut.i"
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 @pytest.fixture(scope="module")
@@ -15,12 +14,8 @@ def fe():
     return importlib.import_module("6dpose_b200.frontend")
 
 
-@pytest.mark.skipif(not os.path.exists(REF_LUT), reason="/root/reference not mounted")
 def test_normal_lut_equals_reference_table(fe):
-    body = open(REF_LUT).read()
-    body = body[body.index("{"):]
-    nums = np.array([int(x) for x in re.findall(r"\d+", body)], np.uint8)[:8000].reshape(20, 20, 20)
-    assert np.array_equal(fe.normal_lut(), nums)
+    assert np.array_equal(fe.normal_lut(), np.load(os.path.join(GOLD, "reference_tables.npz"))["normal_lut"])
 
 
 def naive_hysteresis(mag, angle, thr):

@@ -1,6 +1,6 @@
-"""Pinning of the oracle: (1) against the reference's own linemodLevelup.cpp compiled unmodified
-(oracle/_ref, when built), (2) against the committed golden vectors that code produced on the
-reference's fixture frame and template banks (tests/golden/make_golden.py)."""
+"""Pinning of the oracle against the committed golden vectors that the reference's own linemodLevelup.cpp, compiled
+unmodified (oracle/_ref), produced on the reference's fixture frame and template banks and on synthetic cases
+(tests/golden/make_golden.py)."""
 import importlib
 import os
 
@@ -40,11 +40,11 @@ def test_oracle_reproduces_the_reference_golden_vectors(oracle):
 def load_allscales_full():
     """The reference's own large-bank invocation (linemodLevelup/test.cpp:174-181): Detector() = 63 features, T = {5, 8},
     ALL 2989 templates of test/case1/allScales, threshold 80; plus threshold 75 (61 912 coarse candidates)."""
-    b = np.load(os.path.join(GOLD, "bank_allScales_full.npz"))
-    packed = dict(class_begin=b["class_begin"], tmeta=b["tmeta"].astype(np.int32), feats=b["feats"].astype(np.int32))
+    from oracle import golden
+    packed, T = golden.allscales_full_bank()
     exp = np.load(os.path.join(GOLD, "expected_allScales_full.npz"))
     cases = [(k.split("_")[0], float(k.split("_")[1]), exp[k], exp[k + "_stats"]) for k in exp.files if not k.endswith("_stats")]
-    return packed, b["T"].tolist(), cases
+    return packed, T, cases
 
 
 def test_oracle_reproduces_the_full_allscales_golden_vectors(oracle):
@@ -66,37 +66,47 @@ def test_golden_top_match_sits_on_the_ground_truth_box():
     assert abs(int(top["x"]) - 331) <= 4 and abs(int(top["y"]) - 130) <= 4
 
 
-ref = pytest.importorskip("oracle.ref")
-
-
-@pytest.mark.skipif(not ref.available(), reason="oracle/_ref not built (needs /root/reference)")
-@pytest.mark.parametrize("T,W,H,nf,n,thr", [
+# synthetic cases on which the compiled reference (oracle/_ref) recorded its results in expected_synth.npz
+SYNTH_CASES = [
     ([4, 8], 640, 480, 150, 70, 75.0), ([5, 8], 640, 480, 127, 50, 70.0), ([5, 8], 640, 480, 63, 50, 70.0),
     ([8], 320, 240, 40, 35, 60.0), ([2, 4, 8], 640, 512, 96, 35, 70.0), ([4, 8], 320, 256, 32, 3, -1.0),
-])
-def test_oracle_equals_compiled_reference(oracle, synth, T, W, H, nf, n, thr):
+]
+
+
+def synth_case(synth, T, W, H, nf, n, thr):
     bank = synth.synth_bank(n, num_features=nf, levels=len(T), seed=21, class_ids=("01_template", "02_template"))
     q, _ = synth.synth_frame(W, H, levels=len(T), seed=9, bank=bank, plant=6, T=T)
-    packed = bank.pack(bank.class_ids(), 2 * len(T))
-    a = oracle.match(q, T, packed, thr)
-    b = ref.match(q, T, packed, thr)
-    assert len(b) > 0 and np.array_equal(a, b)
+    return q, bank.pack(bank.class_ids(), 2 * len(T))
 
 
-@pytest.mark.skipif(not ref.available(), reason="oracle/_ref not built (needs /root/reference)")
-def test_similarity_lut_equals_the_compiled_reference_table(oracle):
-    assert np.array_equal(oracle.similarity_lut(), ref.similarity_lut())
+def synth_key(T, W, H, nf, n, thr):
+    return "T%s_%dx%d_f%d_n%d_thr%g" % ("-".join(str(t) for t in T), W, H, nf, n, thr)
 
 
-@pytest.mark.skipif(not ref.available(), reason="oracle/_ref not built (needs /root/reference)")
-def test_reference_assertion_matches_oracle_error(oracle, synth):
+def malformed_case(synth):
+    """A bank whose level-1 colour template lost features: the reference's CV_Assert fires on it."""
     T = [4, 8]
     bank = synth.synth_bank(4, num_features=150, levels=2, seed=8)
     bank.classes["01_template"][2][2].features = bank.classes["01_template"][2][2].features[:10]
     q, _ = synth.synth_frame(320, 256, levels=2, seed=6)
-    packed = bank.pack(bank.class_ids(), 4)
-    with pytest.raises(RuntimeError):
-        ref.match(q, T, packed, 80.0)
+    return q, T, bank.pack(bank.class_ids(), 4)
+
+
+@pytest.mark.parametrize("T,W,H,nf,n,thr", SYNTH_CASES)
+def test_oracle_equals_compiled_reference(oracle, synth, T, W, H, nf, n, thr):
+    q, packed = synth_case(synth, T, W, H, nf, n, thr)
+    want = np.load(os.path.join(GOLD, "expected_synth.npz"))[synth_key(T, W, H, nf, n, thr)]
+    a = oracle.match(q, T, packed, thr)
+    assert len(want) > 0 and np.array_equal(a, want)
+
+
+def test_similarity_lut_equals_the_compiled_reference_table(oracle):
+    assert np.array_equal(oracle.similarity_lut(), np.load(os.path.join(GOLD, "reference_tables.npz"))["similarity_lut"])
+
+
+def test_reference_assertion_matches_oracle_error(oracle, synth):
+    q, T, packed = malformed_case(synth)
+    assert bool(np.load(os.path.join(GOLD, "expected_synth.npz"))["malformed_bank_raises"])   # the compiled reference raised
     with pytest.raises(RuntimeError):
         oracle.match(q, T, packed, 80.0)
 

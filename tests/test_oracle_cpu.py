@@ -1,13 +1,12 @@
 """CPU tests of the oracle (oracle/lm_oracle.cpp): against an independent numpy restatement of the
-same reference functions on small cases, against the reference's own tables when /root/reference is
-mounted, and against the committed golden fixtures."""
+same reference functions on small cases, against the reference's own tables (tests/golden/reference_tables.npz),
+and against the committed golden fixtures."""
 import os
-import re
 
 import numpy as np
 import pytest
 
-REF = "/root/reference/linemodLevelup/linemodLevelup.cpp"
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 # ---- a second, deliberately naive restatement (numpy + Python loops), small cases only ----------
@@ -115,13 +114,7 @@ def np_match(quantized, T, bank, class_ids, threshold):
 def test_similarity_lut_rule_matches_reference_table(oracle):
     lut = oracle.similarity_lut()
     assert set(np.unique(lut)) == {0, 1, 4}
-    if not os.path.exists(REF):
-        pytest.skip("/root/reference not mounted (the table was compared when it was)")
-    lines = open(REF).read().split("\n")
-    active = [ln for ln in lines if ln.startswith("CV_DECL_ALIGNED(16) static const unsigned char SIMILARITY_LUT")]
-    assert len(active) == 1
-    nums = [int(v) for v in re.search(r"\{(.*)\}", active[0]).group(1).split(",")]
-    assert lut.tolist() == nums
+    assert lut.tolist() == np.load(os.path.join(GOLD, "reference_tables.npz"))["similarity_lut"].tolist()
 
 
 @pytest.mark.parametrize("T,H,W", [(4, 32, 48), (5, 40, 80), (8, 64, 64), (2, 16, 32)])

@@ -5,7 +5,7 @@ poseRefine().process(...) / getR / getT :363-368).
 The script lives in the reference checkout, which is mounted in the build container only and must not be copied, so the
 acceptance run is split in two halves that meet in a committed call trace (tests/golden/driver_trace.npz):
 
-  * here (no GPU, /root/reference mounted): tools/run_reference_driver.py executes the UNMODIFIED script against
+  * here (no GPU, reference checkout present): tools/run_reference_driver.py executes the UNMODIFIED script against
     `linemodLevelup_pybind` with the C-ABI handles replaced by oracle-backed stand-ins (test infrastructure: the CPU
     restatement + oracle/icp_oracle.py).  This checks the Python surface the script drives -- constructor, readClasses,
     match with its keyword, Match attributes, poseRefine surface, dtypes -- and that the recorded trace still equals the
@@ -24,7 +24,8 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden", "driver_trace.npz")
-REF = "/root/reference"
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+REF = importlib.import_module("run_reference_driver").REF   # the checkout the harness runs the script from
 TOL = 1e-4
 
 
@@ -128,7 +129,7 @@ def trace_arrays(trace):
     return out
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "linemodLevelup")), reason="reference checkout not mounted")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "linemodLevelup")), reason="reference checkout not found")
 def test_unmodified_driver_runs_against_the_module_surface(oracle):
     trace = run_script_with_oracle_backends()
     mc = trace["match_calls"][0]
@@ -159,8 +160,8 @@ def test_recorded_driver_calls_through_the_cuda_backend(tmp_path):
     gold = np.load(GOLD)
     bk = importlib.import_module("6dpose_b200.bank")
     mod = importlib.import_module("linemodLevelup_pybind")
-    b = np.load(os.path.join(ROOT, "tests", "golden", "bank_allScales_full.npz"))   # the bank the recorded run read
-    packed = dict(class_begin=b["class_begin"], tmeta=b["tmeta"].astype(np.int32), feats=b["feats"].astype(np.int32))
+    from oracle import golden
+    packed, _ = golden.allscales_full_bank()   # the bank the recorded run read
     bank = bk.TemplateBank()
     bank.classes["06_template"] = bk.PackedPyramids(packed["tmeta"], packed["feats"], 2)   # one class: feat_begin is class-local
     bank.write_packed("06_template", str(tmp_path / "06_template.lmb"), 2)

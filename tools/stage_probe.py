@@ -29,11 +29,9 @@ def main():
     lib = importlib.import_module("6dpose_b200._lib")
     synth = importlib.import_module("6dpose_b200.synth")
     if args.real:
-        g = os.path.join(ROOT, "tests", "golden")
-        b = np.load(os.path.join(g, "bank_allScales_full.npz"))
-        packed = dict(class_begin=b["class_begin"], tmeta=b["tmeta"].astype(np.int32), feats=b["feats"].astype(np.int32))
-        T = b["T"].tolist()
-        fr = np.load(os.path.join(g, "frames_case1.npz"))
+        from oracle import golden
+        packed, T = golden.allscales_full_bank()
+        fr = np.load(os.path.join(golden.GOLD, "frames_case1.npz"))
         frames = [[[fr["full_l%d_m%d" % (l, m)] for m in range(2)] for l in range(2)]]
     else:
         T = [4, 8]
