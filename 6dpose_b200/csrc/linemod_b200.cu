@@ -121,23 +121,15 @@ struct lm_detector {
   std::vector<uint8_t> safe;         // per template: refinement never skips a feature (LL.cpp:1394)
   uint8_t* d_safe = nullptr;
   uint16_t* d_galign = nullptr;      // [G][S][16] feature counts per (address & 15) group
-  // refinement filter (k_refine_filter) on the first refined level lr = L - 2: column-major H-planes + descriptors
-  bool filter_on = true;             // LINEMOD_B200_FILTER=0 switches it off (profiling / A-B runs)
+  // refinement filter (k_refine_filter_w) on the first refined level lr = L - 2: column-major H-planes + descriptors
   bool filter_ok = false;            // the current frame size / bank allow it
-  bool k2_small_global = false;      // LINEMOD_B200_K2_SMALL_GLOBAL=1: small shards read the planes through L1 (no staging)
-  bool k2_smem = true;               // LINEMOD_B200_K2_SMEM=0: bit-planes read from global memory / L1 (no staging, no shared memory held)
-  bool k2_split = true;              // LINEMOD_B200_K2_SPLIT=0: one warp per coarse-scan task whatever the shard
-  bool planes_direct = true;         // LINEMOD_B200_PLANES_DIRECT=0: K1 always writes byte linear memories, k_refine_prep derives the planes
   int last_planes_level = -1;        // level the last K1 built in planes mode (its byte linear memories are stale)
-  bool bits_exact = true;            // LINEMOD_B200_BITS_EXACT=0: survivors go to the byte-wise k_refine instead
-  int filter_variant = 0;            // 0: warp per candidate (k_refine_filter_w), 1: 8 lanes per candidate (k_refine_filter)
   uint32_t* d_rp = nullptr; size_t rp_words = 0; int rp_nyb = 0;
   uint32_t* d_rdesc = nullptr;       // per feature of level lr, grouped per template, padded to multiples of 32
   uint8_t* d_rlab = nullptr;         // label per descriptor (8 = padding): k_refine_bits derives the neighbour planes
   bool shard_all_eligible = false;   // every template of the shard is taken by the filter (no byte-wise refinement)
   uint32_t* d_surv2 = nullptr;       // candidates of the templates the filter does not take
-  int2* d_rfeat = nullptr;           // per template: first descriptor, count
-  std::vector<int2> h_rfeat;
+  std::vector<int2> h_rfeat;         // per template: first descriptor, count (feeds h_finfo)
   int4* d_finfo = nullptr;           // per work item of the shard: first descriptor, count, width | height << 16,
                                      // flags | need << 8 (need: for the threshold of the call, see filter_thresholds)
   std::vector<int4> h_finfo;         // .w = flags only
@@ -274,22 +266,6 @@ extern "C" int lm_create(int device, int n_levels, const int* T, lm_detector** o
   memset(d->h_counters, 0, 8 * sizeof(unsigned long long));
   CU(cudaMalloc(&d->d_queue, 4 * sizeof(int)));
   CU(cudaMemset(d->d_queue, 0, 4 * sizeof(int)));
-  {
-    const char* f = getenv("LINEMOD_B200_FILTER");
-    d->filter_on = !(f && f[0] == '0');
-    const char* fkg = getenv("LINEMOD_B200_K2_SMALL_GLOBAL");
-    d->k2_small_global = fkg && fkg[0] == '1';
-    const char* fkm = getenv("LINEMOD_B200_K2_SMEM");
-    d->k2_smem = !(fkm && fkm[0] == '0');
-    const char* fks = getenv("LINEMOD_B200_K2_SPLIT");
-    d->k2_split = !(fks && fks[0] == '0');
-    const char* fpd = getenv("LINEMOD_B200_PLANES_DIRECT");
-    d->planes_direct = !(fpd && fpd[0] == '0');
-    const char* fb = getenv("LINEMOD_B200_BITS_EXACT");
-    d->bits_exact = !(fb && fb[0] == '0');
-    const char* fv = getenv("LINEMOD_B200_FILTER_VARIANT");
-    d->filter_variant = (fv && fv[0] == '1') ? 1 : 0;
-  }
   *out = d;
   return LM_OK;
 }
@@ -321,7 +297,7 @@ extern "C" void lm_destroy(lm_detector* d) {
   cudaFree(d->d_mask); cudaFree(d->d_raw); cudaFree(d->d_cnt); cudaFree(d->d_off);
   cudaFree(d->d_res_own); cudaFree(d->d_counters);
   cudaFree(d->d_finfo); cudaFree(d->d_rlab); cudaFree(d->d_surv2);
-  cudaFree(d->d_rp); cudaFree(d->d_rdesc); cudaFree(d->d_rfeat); cudaFree(d->d_cand); cudaFree(d->d_surv); cudaFree(d->d_queue);
+  cudaFree(d->d_rp); cudaFree(d->d_rdesc); cudaFree(d->d_cand); cudaFree(d->d_surv); cudaFree(d->d_queue);
   cudaFreeHost(d->h_counters); cudaFreeHost(d->h_res);
   cudaFree(d->d_post_info); cudaFree(d->d_post_out); cudaFree(d->d_post_counts); cudaFree(d->d_post_live);
   cudaFreeHost(d->h_post_out); cudaFreeHost(d->h_post_counts);
@@ -617,7 +593,7 @@ static int prepare_bank(lm_detector* d) {
     CU(cudaMalloc(&d->d_galign, galign.size() * sizeof(uint16_t)));
     CU(cudaMemcpyAsync(d->d_galign, galign.data(), galign.size() * sizeof(uint16_t), cudaMemcpyHostToDevice, d->stream));
   }
-  // refinement filter (k_refine_filter) on the first refined level: column-major H-planes [M*8*T*T][nyb][Wd] and one
+  // refinement filter (k_refine_filter_w) on the first refined level: column-major H-planes [M*8*T*T][nyb][Wd] and one
   // descriptor per feature = plane word offset (incl. x / T) : 23 | y / T : 9.  Eligible templates ("safe", so that
   // the 16x16 patch of every feature is a true 2-D window of the level, and at most 511 features at that level) get
   // bit 1 of their flag byte; the others go to k_refine unfiltered.
@@ -625,7 +601,7 @@ static int prepare_bank(lm_detector* d) {
   std::vector<uint32_t> rdesc;
   std::vector<uint8_t> rlab;
   std::vector<int2> rfeat((size_t)d->G, make_int2(0, 0));
-  if (d->filter_on && d->L >= 2) {
+  if (d->L >= 2) {
     const int lr = d->L - 2;
     const LevelHost& lv = d->lv[lr];
     const int T = lv.T, T2 = T * T;
@@ -667,15 +643,12 @@ static int prepare_bank(lm_detector* d) {
   }
   d->h_rfeat = rfeat;
   cudaFree(d->d_rdesc); d->d_rdesc = nullptr;
-  cudaFree(d->d_rfeat); d->d_rfeat = nullptr;
   cudaFree(d->d_rlab); d->d_rlab = nullptr;
   if (d->filter_ok) {
     CU(cudaMalloc(&d->d_rlab, std::max<size_t>(rlab.size(), 1)));
     if (!rlab.empty()) CU(cudaMemcpyAsync(d->d_rlab, rlab.data(), rlab.size(), cudaMemcpyHostToDevice, d->stream));
     CU(cudaMalloc(&d->d_rdesc, std::max<size_t>(rdesc.size(), 1) * 4));
-    CU(cudaMalloc(&d->d_rfeat, std::max<size_t>(rfeat.size(), 1) * sizeof(int2)));
     if (!rdesc.empty()) CU(cudaMemcpyAsync(d->d_rdesc, rdesc.data(), rdesc.size() * 4, cudaMemcpyHostToDevice, d->stream));
-    if (!rfeat.empty()) CU(cudaMemcpyAsync(d->d_rfeat, rfeat.data(), rfeat.size() * sizeof(int2), cudaMemcpyHostToDevice, d->stream));
   }
   cudaFree(d->d_safe);
   d->d_safe = nullptr;
@@ -782,7 +755,7 @@ static int host_min_kept_raw(float threshold, int nfeat) {
 }
 
 // finfo[w].w = flags | need << 8 for this threshold: need = number of features whose label bit must be set at some cell
-// of the patch for the candidate to be able to reach raw_keep (see k_refine_filter).
+// of the patch for the candidate to be able to reach raw_keep (see k_refine_filter_w).
 static int filter_thresholds(lm_detector* d, float threshold) {
   if (!d->filter_ok || !d->d_finfo || d->h_finfo.empty()) return LM_OK;
   if (d->finfo_valid && memcmp(&threshold, &d->finfo_threshold, sizeof(float)) == 0) return LM_OK;
@@ -1054,7 +1027,6 @@ static void plan_k1(lm_detector* d, int planes_level, bool with_bit_planes, K1Pl
       int pseg = 4;
       for (int c : {32, 16, 8})
         if (lv.Wd % c == 0 && lv.T * lv.T * c <= 128) { pseg = c; break; }
-      if (const char* e = getenv("LINEMOD_B200_PSEG")) { const int v = atoi(e); if (v >= 4 && v % 4 == 0 && lv.Wd % v == 0) pseg = v; }
       p.lv[l].pseg = pseg;
       const size_t wpp = (size_t)((pseg * lv.T + lv.T + 3 + 4) & ~3);
       need = wpp * (size_t)(2 * (16 * lv.T + lv.T - 1) + 16 * lv.T);
@@ -1098,11 +1070,9 @@ static int launch_k1(lm_detector* d, const K1Plan& k, int first_block, int n_blo
 
 // Which refinement path the current bank / shard / frame size take (see enqueue_stages).
 static bool use_filter(const lm_detector* d) { return d->filter_ok && d->d_rp != nullptr && d->d_finfo != nullptr; }
-static bool use_bits(const lm_detector* d) { return use_filter(d) && d->L == 2 && d->filter_variant == 0 && d->bits_exact; }
+static bool use_bits(const lm_detector* d) { return use_filter(d) && d->L == 2; }
 // level built in planes mode by K1, or -1: only when nothing reads that level's byte linear memories
-static int planes_level(const lm_detector* d) {
-  return (use_bits(d) && d->shard_all_eligible && d->planes_direct) ? d->L - 2 : -1;
-}
+static int planes_level(const lm_detector* d) { return use_bits(d) && d->shard_all_eligible ? d->L - 2 : -1; }
 
 // Enqueue every GPU stage of one frame on the detector's stream; no host synchronisation.
 static int enqueue_stages(lm_detector* d, float threshold, bool refine_only) {
@@ -1160,7 +1130,7 @@ static int enqueue_stages(lm_detector* d, float threshold, bool refine_only) {
       bp.queue = d->d_queue;
       bp.ticket = reinterpret_cast<int*>(d->d_counters + 3);
       const size_t plane_bytes = ((size_t)bp.bp_words * 4 + 15) & ~(size_t)15;
-      bool smem = plane_bytes <= LM_BITS_SMEM_LIMIT && d->k2_smem;
+      const bool smem = plane_bytes <= LM_BITS_SMEM_LIMIT;
       // tasks of 32 words (full rounds + packed remainders).  One task per warp (or per TEAM of S warps when the shard has
       // fewer tasks than the GPU has warp slots: the team deals the task's features, so the kernel's latency follows the
       // shard) and one round per CTA: the CTA size follows the shard, so a small shard spreads over all SMs.
@@ -1169,12 +1139,9 @@ static int enqueue_stages(lm_detector* d, float threshold, bool refine_only) {
       const long long tasks = (long long)d->n_items_bits * (low.nwords / 32) +
                               ((long long)d->n_items_bits * (low.nwords % 32) + 31) / 32;
       const long long slots = (long long)d->sm_count * (LM_PACK_THREADS / 32);
-      // optional (LINEMOD_B200_K2_SMALL_GLOBAL=1): a small shard reads the planes through L1 instead of staging them --
-      // same latency measured (22 vs 23 us at 1/8 of the bank), no shared memory held; no throughput gain measured at N=8
-      if (d->k2_split && d->k2_small_global && tasks * 4 <= slots) smem = false;
       const size_t part_room = LM_K2_SMEM_MAX - (smem ? plane_bytes : (size_t)LM_K2_SMEM_MAX - 64 * 1024);
       int S = 1;
-      while (d->k2_split && S < 8 && tasks * (S * 2) <= slots) {
+      while (S < 8 && tasks * (S * 2) <= slots) {
         const int S2 = S * 2;
         long long w2 = (tasks * S2 + d->sm_count - 1) / d->sm_count;
         w2 = std::min<long long>(LM_PACK_THREADS / 32, std::max<long long>(std::max(4, S2), (w2 + S2 - 1) / S2 * S2));
@@ -1250,15 +1217,12 @@ static int enqueue_stages(lm_detector* d, float threshold, bool refine_only) {
   if (d->timing && !refine_only) CU(cudaEventRecord(d->ev[4], st));
   if (filter) {
     FilterParams fp;
-    fp.rp = d->d_rp; fp.Wd = lref.Wd; fp.nyb = d->rp_nyb;
-    fp.rdesc = d->d_rdesc; fp.rfeat = d->d_rfeat; fp.finfo = d->d_finfo; fp.flags = d->d_safe;
-    fp.tslot = d->d_tslot; fp.work = d->d_work; fp.S = d->S; fp.M = d->M; fp.L = d->L;
+    fp.rp = d->d_rp; fp.Wd = lref.Wd;
+    fp.rdesc = d->d_rdesc; fp.finfo = d->d_finfo;
     fp.low = level_dev(low); fp.ref = level_dev(lref);
     fp.cand = d->d_cand; fp.off = d->d_off; fp.n_work = n_work; fp.cand_cap = (int)d->cand_cap;
-    fp.threshold = threshold;
     fp.surv = d->d_surv; fp.surv2 = bits_mode ? d->d_surv2 : nullptr; fp.queue = d->d_queue; fp.counters = d->d_counters;
-    if (d->filter_variant == 0) CU(launch_pdl(k_refine_filter_w, dim3((unsigned)(d->sm_count * LM_FILTER_MIN_CTAS)), dim3(256), 0, st, fp));
-    else CU(launch_pdl(k_refine_filter, dim3((unsigned)(d->sm_count * 4)), dim3(256), 0, st, fp));
+    CU(launch_pdl(k_refine_filter_w, dim3((unsigned)(d->sm_count * LM_FILTER_MIN_CTAS)), dim3(256), 0, st, fp));
     ++d->launches;
   }
   if (d->timing && !refine_only) CU(cudaEventRecord(d->ev[5], st));

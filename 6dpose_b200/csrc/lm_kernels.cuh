@@ -9,7 +9,7 @@
 //                                                                           LL.cpp:1284-1354, 1435-1534, 1836-1852
 //   k_scan_counts      <- candidates.push_back ordering (deterministic offsets)
 //   k_refine_prep      <- the candidate list in the reference's pre-sort order
-//   k_refine_filter(_w) + k_refine_bits <- similarityLocal(_64) + best-cell search + remove_if, bit-sliced: an exact
+//   k_refine_filter_w + k_refine_bits <- similarityLocal(_64) + best-cell search + remove_if, bit-sliced: an exact
 //                         upper-bound filter, then exact scoring of its survivors      LL.cpp:1366-1428, 1855-1938
 //   k_refine<split>    <- the same, byte-wise (templates / pyramids the bit-sliced path does not take)
 #pragma once
@@ -486,9 +486,7 @@ __device__ __forceinline__ void vc_add8(uint32_t (&c)[8], const uint32_t (&x)[8]
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-#ifndef LM_PACK_THREADS
 #define LM_PACK_THREADS 768
-#endif
 
 // exclusive scan of the per-template candidate counts -> off[], result header and counters reset for k_refine,
 // counts re-zeroed for the next frame's atomics.  Whole CTA.
@@ -514,9 +512,9 @@ __device__ __forceinline__ void scan_counts_block(int32_t* __restrict__ cnt, int
     hdr->shard = shard;
     counters[0] = 0ull;  // k_refine accumulates into them
     counters[1] = 0ull;
-    counters[4] = 0ull;  // k_refine_filter: features x candidates it dropped, plane words it read
+    counters[4] = 0ull;  // k_refine_filter_w: features x candidates it dropped, plane words it read
     counters[5] = 0ull;
-    queue[0] = 0;        // k_refine_filter: next candidate, survivors appended (two lists)
+    queue[0] = 0;        // k_refine_filter_w: next candidate, survivors appended (two lists)
     queue[1] = 0;
     queue[2] = 0;
   }
@@ -1079,39 +1077,26 @@ __global__ void __launch_bounds__(256) k_refine_prep(PrepParams p) {
 }
 
 // --------------------------------------------------------------------------------------------
-// k_refine_filter: exact upper-bound test in front of the refinement, bit-sliced.
+// k_refine_filter_w: exact upper-bound test in front of the refinement, bit-sliced.
 //
 // similarityLocal adds, per feature, 4 where the feature's label bit is set in the spread mask (H), else at most 1
 // (LL.cpp:1121 table; lm_response).  So for every cell of the 16x16 patch  raw <= 4*CH + (nf - CH) = 3*CH + nf  with CH =
 // number of features whose H bit is set at that cell.  A candidate survives remove_if (LL.cpp:1935-1937) only if its best
 // cell reaches raw_keep, i.e. only if SOME cell has CH >= need = ceil((raw_keep - nf) / 3).  Candidates without such a cell
-// are dropped here without ever touching the byte linear memories; the others (a few percent) go on to k_refine, which
-// computes them exactly as before -- the filter never changes a result, it only removes work.
-//
-// Eight lanes own one candidate (four candidates per warp): lane k holds patch columns k and k + 8 as the two halves of
-// a 32-bit word (16 rows each) and counts CH for its 32 cells in a 9-bit vertical counter (carry-save adders, 8 features
-// per step).  Per feature and lane: two 32-bit loads from the column-major H-planes (k_refine_prep), two shifts, one
-// byte-permute.  Every 32 features the cells that cannot reach `need` any more (CH + remaining < need) are found with a
-// bit-sliced compare; a lane without live cells stops loading, a candidate without live cells is dropped at once.  The
-// four groups of a warp run independently: each fetches its next candidate from a global counter when it is done.
+// are dropped here without ever touching the byte linear memories; the others (a few percent) go on to the exact
+// refinement (k_refine_bits / k_refine) -- the filter never changes a result, it only removes work.
 // --------------------------------------------------------------------------------------------
 struct FilterParams {
   const uint32_t* rp;      // H-planes of the filtered level
-  int Wd, nyb;
+  int Wd;
   const uint32_t* rdesc;   // per feature (own order, grouped per template): plane word offset incl. x / T : 23 | y / T : 9
-  const int2* rfeat;       // per template: first descriptor, number of features of the level (all modalities)
-  const int4* finfo;       // per WORK ITEM of the shard: the same + width | height << 16 of the level's template + flags
-  const uint8_t* flags;    // per template: bit 0 = "safe" (k_refine's fast path), bit 1 = the filter may take it
-  const TSlot* tslot;
-  const int32_t* work;
-  int S, M, L;
+  const int4* finfo;       // per WORK ITEM of the shard (layout below); flags bit 1 = the filter may take the template
   LevelDev low, ref;       // lowest level (cell -> pixel), filtered level (clamp, patch origin)
   const uint2* cand;
   const int32_t* off;
   int n_work, cand_cap;
-  float threshold;
   uint32_t* surv;          // survivors (candidate indices), unordered
-  uint32_t* surv2;         // optional second list: candidates of templates the filter does not take (k_refine_filter_w)
+  uint32_t* surv2;         // optional second list: candidates of templates the filter does not take
   int* queue;              // [0] next candidate, [1] survivors, [2] entries of surv2
   unsigned long long* counters;  // [4] features x candidates dropped here, [5] plane words read
 };
@@ -1137,138 +1122,15 @@ __device__ __forceinline__ void vc_add8n(uint32_t (&c)[NB], const uint32_t (&x)[
 
 #define LM_FILTER_BITS 9   // CH <= 511 features of the filtered level
 
-__global__ void __launch_bounds__(256, 4) k_refine_filter(FilterParams p) {
-  lm_pdl_wait();
-  const int lane = threadIdx.x & 31, grp = lane >> 3, gl = lane & 7;
-  const unsigned gmask = 0xFFu << (grp * 8);
-  const int total = min(p.off[p.n_work], p.cand_cap);
-  const int lr = p.L - 2;
-  int c = -1, nf = 0, first = 0, need = 0, i = 0, base0 = 0, cy = 0;
-  bool exhausted = false, lane_alive = false;
-  uint32_t ch[LM_FILTER_BITS];
-#pragma unroll
-  for (int b = 0; b < LM_FILTER_BITS; ++b) ch[b] = 0u;
-  unsigned words_read = 0, dropped_feats = 0;
-
-  for (;;) {
-    // ---- groups without a candidate fetch the next one (one atomic per warp and round)
-    const bool want = c < 0 && !exhausted;
-    const unsigned fetch = __ballot_sync(0xffffffffu, want && gl == 0);
-    if (fetch) {
-      const int leader = __ffs(fetch) - 1;
-      int basec = 0;
-      if (lane == leader) basec = atomicAdd(p.queue, __popc(fetch));
-      basec = __shfl_sync(0xffffffffu, basec, leader);
-      if (want) {
-        const int cc = basec + __popc(fetch & ((1u << (grp * 8)) - 1u));
-        if (cc >= total) {
-          exhausted = true;
-        } else {
-          const uint2 e = __ldcg(p.cand + cc);
-          const int w = (int)e.x, j = (int)e.y;
-          const int g = p.work[w];
-          bool pass = true;  // hand the candidate to k_refine unfiltered
-          if (p.flags[g] & 2) {
-            const int2 rf = p.rfeat[g];
-            nf = rf.y;
-            first = rf.x;
-            const int raw_keep = lm_min_kept_raw(p.threshold, nf);
-            need = raw_keep - nf;
-            need = need > 0 ? (need + 2) / 3 : 0;
-            if (need > nf) {  // nothing can be kept (LL.cpp:1935-1937 would drop whatever the patch holds)
-              if (gl == 0) dropped_feats += (unsigned)nf;
-              pass = false;
-            } else if (need > 0) {
-              // patch origin of the candidate at the filtered level (LL.cpp:1871-1880, 1380-1381)
-              const TSlot t0 = p.tslot[(size_t)g * p.S + lr * p.M];
-              const int T = p.ref.T, border = 8 * T;
-              int x = (j % p.low.Wd) * p.low.T + p.low.off;
-              int y = (j / p.low.Wd) * p.low.T + p.low.off;
-              x = x * 2 + 1;
-              y = y * 2 + 1;
-              x = max(x, border); y = max(y, border);
-              x = min(x, p.ref.cols - (t0.w & 0xFFFF) - border);
-              y = min(y, p.ref.rows - (int)((unsigned)t0.w >> 16) - border);
-              base0 = x / T - 8 + gl;
-              cy = y / T - 8;
-              i = 0;
-              lane_alive = true;
-#pragma unroll
-              for (int b = 0; b < LM_FILTER_BITS; ++b) ch[b] = 0u;
-              c = cc;
-              pass = false;
-            }
-          }
-          if (pass && gl == 0) p.surv[atomicAdd(p.queue + 1, 1)] = (uint32_t)cc;
-        }
-      }
-    }
-    if (__all_sync(0xffffffffu, c < 0 && exhausted)) break;
-
-    // ---- one step: 8 features of every group that holds a candidate
-    const bool act = c >= 0;
-    uint32_t xh[8];
-#pragma unroll
-    for (int u = 0; u < 8; ++u) {
-      uint32_t h = 0u;
-      if (act && lane_alive && i + u < nf) {
-        const uint32_t d = __ldg(p.rdesc + first + i + u);
-        const int py0 = cy + (int)(d >> 23);
-        const uint32_t* __restrict__ ptr = p.rp + (d & 0x7FFFFFu) + (py0 >> 4) * p.Wd + base0;
-        const uint32_t sft = (uint32_t)py0 & 15u;
-        h = __byte_perm(__ldg(ptr) >> sft, __ldg(ptr + 8) >> sft, 0x5410);
-        words_read += 2;
-      }
-      xh[u] = h;
-    }
-    vc_add8n<LM_FILTER_BITS>(ch, xh);
-    if (act) {
-      i += 8;
-      const bool end = i >= nf;
-      if (end || (i & 31) == 0) {
-        // cells that can still reach `need`: CH >= need - (features not yet added)
-        const int thr_now = need - (nf - min(i, nf));
-        uint32_t alive_cells = 0xffffffffu;
-        if (thr_now > 0) {
-          uint32_t gt = 0u, eq = 0xffffffffu;
-#pragma unroll
-          for (int b = LM_FILTER_BITS - 1; b >= 0; --b) {
-            const uint32_t tb = 0u - (((uint32_t)thr_now >> b) & 1u);
-            gt |= eq & ch[b] & ~tb;
-            eq &= ~(ch[b] ^ tb);
-          }
-          alive_cells = gt | eq;
-        }
-        lane_alive = alive_cells != 0u;
-        const unsigned g_alive = __ballot_sync(gmask, lane_alive);
-        if (g_alive == 0u) {
-          if (gl == 0) dropped_feats += (unsigned)nf;  // the reference's work for it (algorithmic bytes / 256)
-          c = -1;
-        } else if (end) {
-          if (gl == 0) p.surv[atomicAdd(p.queue + 1, 1)] = (uint32_t)c;
-          c = -1;
-        }
-      }
-    }
-  }
-  words_read = __reduce_add_sync(0xffffffffu, words_read);
-  dropped_feats = __reduce_add_sync(0xffffffffu, dropped_feats);
-  if (lane == 0 && (words_read | dropped_feats)) {
-    atomicAdd(p.counters + 4, (unsigned long long)dropped_feats);
-    atomicAdd(p.counters + 5, (unsigned long long)words_read);
-  }
-}
-
-
-// k_refine_filter_w: the same test with ONE WARP per candidate (the default; LINEMOD_B200_FILTER_VARIANT=1 selects the
-// kernel above).  The four 8-lane groups of the warp work on the SAME 16x16 patch and deal the features between them: of
-// every 32 consecutive features group q adds features 8q .. 8q+7 into its own partial counter, so a candidate is a chain
-// of nf / 32 steps instead of nf / 8 (a chain four times shorter: what matters when the candidates are fewer than the
-// machine has lanes, e.g. a 1/8 template shard).  Lane L decodes descriptor L of the step once (word offset and shift
-// packed in one register) and the lanes of group q pick theirs up by shuffle; control flow is warp-uniform.  The partial
-// counters meet (bit-sliced adds across the groups, two butterfly steps) at two check points -- after about half and
-// three quarters of the features -- where cells, lanes and whole candidates that can no longer reach `need` are dropped,
-// and at the end.
+// One warp per candidate.  Lane k of an 8-lane group holds patch columns k and k + 8 as the two halves of a 32-bit word (16
+// rows each) and counts CH for its 32 cells in a 9-bit vertical counter (carry-save adders, 8 features per step).  The
+// four 8-lane groups of the warp work on the SAME 16x16 patch and deal the features between them: of every 32 consecutive
+// features group q adds features 8q .. 8q+7 into its own partial counter, so a candidate is a chain of nf / 32 steps
+// (what matters when the candidates are fewer than the machine has lanes, e.g. a 1/8 template shard).  Lane L decodes
+// descriptor L of the step once (word offset and shift packed in one register) and the lanes of group q pick theirs up by
+// shuffle; control flow is warp-uniform.  The partial counters meet (bit-sliced adds across the groups, two butterfly
+// steps) at two check points -- after about half and three quarters of the features -- where cells, lanes and whole
+// candidates that can no longer reach `need` are dropped, and at the end.
 __device__ __forceinline__ void vc_allreduce_groups(uint32_t (&c)[LM_FILTER_BITS]) {
 #pragma unroll
   for (int step = 8; step <= 16; step <<= 1) {
@@ -1302,12 +1164,7 @@ __device__ __forceinline__ const uint32_t* lm_ptr_add(const char* base, uint32_t
   return reinterpret_cast<const uint32_t*>(r);
 }
 
-#ifndef LM_FILTER_MIN_CTAS
 #define LM_FILTER_MIN_CTAS 5
-#endif
-#ifndef LM_FILTER_CHUNK
-#define LM_FILTER_CHUNK 1  // consecutive candidates a warp takes from the queue at a time (2..16 measured: tail imbalance costs more than the L1 reuse buys)
-#endif
 // Layout contract with the host (prepare_bank / prepare_work): every template's descriptors are padded to a multiple of
 // 32 with descriptors that point into an all-zero tail of the plane buffer (so the loop needs no bounds predicate), and
 // finfo[w] = {first descriptor, features of the level, width | height << 16, flags | need << 8} with `need` computed on
@@ -1319,14 +1176,12 @@ __global__ void __launch_bounds__(256, LM_FILTER_MIN_CTAS) k_refine_filter_w(Fil
   const int T = p.ref.T, border = 8 * T;
   const int Wd = p.Wd;
   unsigned words_read = 0, dropped_feats = 0;
-  // A warp takes LM_FILTER_CHUNK consecutive candidates at a time: the list is ordered by template, then cell, so they
-  // mostly share the template (descriptors) and their patches overlap (neighbouring cells) -- what the first one pulled
-  // into L1 serves the others.  The NEXT candidate's cell and per-template record are fetched while the current one is
-  // being counted.
-  int c_base = 0, k_in = 0;
-  if (lane == 0) c_base = atomicAdd(p.queue, LM_FILTER_CHUNK);
-  c_base = __shfl_sync(0xffffffffu, c_base, 0);
-  int c_next = c_base;
+  // A warp takes one candidate at a time from the queue (taking 2..16 consecutive ones, for L1 reuse between neighbouring
+  // cells, was measured slower: the tail imbalance costs more).  The NEXT candidate's cell and per-work-item record are
+  // fetched while the current one is being counted.
+  int c_next = 0;
+  if (lane == 0) c_next = atomicAdd(p.queue, 1);
+  c_next = __shfl_sync(0xffffffffu, c_next, 0);
   uint2 e_next = make_uint2(0u, 0u);
   int4 fi_next = make_int4(0, 0, 0, 0);
   if (c_next < total) {
@@ -1338,12 +1193,8 @@ __global__ void __launch_bounds__(256, LM_FILTER_MIN_CTAS) k_refine_filter_w(Fil
     if (c >= total) break;
     const uint2 e = e_next;
     const int4 fi = fi_next;
-    if (++k_in == LM_FILTER_CHUNK) {
-      k_in = 0;
-      if (lane == 0) c_base = atomicAdd(p.queue, LM_FILTER_CHUNK);
-      c_base = __shfl_sync(0xffffffffu, c_base, 0);
-    }
-    c_next = c_base + k_in;
+    if (lane == 0) c_next = atomicAdd(p.queue, 1);
+    c_next = __shfl_sync(0xffffffffu, c_next, 0);
     if (c_next < total) {
       e_next = __ldcg(p.cand + c_next);
       fi_next = __ldg(p.finfo + e_next.x);
@@ -1503,7 +1354,7 @@ struct RefineParams {
   const uint2* cand;     // ordered candidate list (k_refine_prep)
   int cand_cap;
   const uint16_t* raw;   // [n_work][plane_low] coarse raw scores (read when there is no level to refine)
-  const uint32_t* surv;  // work items: a list of candidate indices written by k_refine_filter, or null: every candidate
+  const uint32_t* surv;  // work items: a list of candidate indices written by k_refine_filter_w, or null: every candidate
   const int* queue;      // queue[surv_slot] = length of that list
   int surv_slot;
   int publish;           // multi-GPU: this is the last kernel of the frame that appends records
@@ -1525,9 +1376,7 @@ struct RefineParams {
 // One lane pair = one row of the 16x16 patch: lane `half` loads the aligned 16-byte chunk (a >> 4) +
 // half; K = word offset of the row start inside the first chunk.  The lane then needs the words
 // K + 2*half .. K + 2*half + 2 of the 8-word pair and gets the ones it lacks from its partner.
-#ifndef LM_REFINE_CHECK
 #define LM_REFINE_CHECK 21  // features between two early-exit tests of the refinement (<= 63)
-#endif
 
 template <int K>
 __device__ __forceinline__ void refine_rows(const uint4* __restrict__ lm128, const uint32_t* __restrict__ fb, int n,
@@ -1560,9 +1409,7 @@ __device__ __forceinline__ void refine_rows(const uint4* __restrict__ lm128, con
   }
 }
 
-#ifndef LM_REFINE_MIN_CTAS
 #define LM_REFINE_MIN_CTAS 4
-#endif
 // kSplit = false: one warp per candidate, exact row-wise early exit (every coarse candidate comes here: no filter).
 // kSplit = true : the work items are the filter's survivors -- few (a few percent of the candidates) and nearly all of
 //   them kept, so the early exit has nothing to skip and ONE warp per candidate would leave the kernel waiting on a
@@ -1585,7 +1432,7 @@ __global__ void __launch_bounds__(256, LM_REFINE_MIN_CTAS) k_refine(RefineParams
   if (p.bp_clear)
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < p.bp_words; i += gridDim.x * blockDim.x) p.bp_clear[i] = 0u;
 
-  // work items: the survivors of k_refine_filter (unordered candidate indices), or every candidate
+  // work items: the survivors of k_refine_filter_w (unordered candidate indices), or every candidate
   const int n_items = p.surv ? min(__ldcg(p.queue + p.surv_slot), total) : total;
   for (int base = blockIdx.x * per_cta; base < n_items; base += gridDim.x * per_cta) {
     const int it = base + (kSplit ? (warp >> 2) : warp);

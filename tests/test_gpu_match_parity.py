@@ -147,31 +147,24 @@ def test_reference_assertion_is_an_error(synth, oracle):
         nat.load_bank(packed, 4)
 
 
-@pytest.mark.parametrize("env", [
-    {"LINEMOD_B200_FILTER": "0"},                                   # no filter: byte-wise refinement of every candidate
-    {"LINEMOD_B200_BITS_EXACT": "0"},                               # filter, survivors refined byte-wise by four warps each
-    {"LINEMOD_B200_FILTER_VARIANT": "1"},                           # 8-lanes-per-candidate filter + byte-wise survivors
-    {"LINEMOD_B200_PLANES_DIRECT": "0"},                            # H-planes derived from the byte linear memories
-    {"LINEMOD_B200_K2_SPLIT": "0"},                                 # one warp per coarse task whatever the shard
-    {"LINEMOD_B200_PLANES_DIRECT": "0", "LINEMOD_B200_K2_SPLIT": "0", "LINEMOD_B200_BITS_EXACT": "0"},
+@pytest.mark.parametrize("T,W,H,nf,n,thr", [
+    ([4, 8], 320, 2080, 150, 140, 75.0),  # 16-bit path
+    ([5, 8], 320, 2640, 63, 70, 70.0),    # the reference's 8-bit (_64) path
 ])
-def test_alternative_kernel_paths_bit_exact(synth, oracle, env, monkeypatch):
-    """Every switchable path (the fallbacks the default path replaced, kept for templates / pyramids it does not take and
-    for A/B runs) gives the oracle's result too.  The switches are read when the handle is created."""
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
-    for T, W, H, nf, n, thr in (([4, 8], 640, 480, 150, 140, 75.0), ([5, 8], 640, 480, 63, 70, 70.0), ([2, 4, 8], 640, 512, 96, 35, 70.0)):
-        bank = synth.synth_bank(n, num_features=nf, levels=len(T), seed=21, class_ids=("01_template", "02_template"))
-        q, _ = synth.synth_frame(W, H, levels=len(T), seed=9, bank=bank, plant=6, T=T)
-        nat, packed = _native(T, bank)
-        got = nat.match_quantized(q, thr)
-        want, st = oracle.match(q, T, packed, thr, want_stats=True)
-        assert len(want) > 0
-        _assert_same(got, want)
-        c = nat.counters()
-        assert c["coarse_candidates"] == int(st["coarse_candidates"])
-        assert c["refine_bytes"] == int(st["refine_byte_adds"])
-        nat.close()
+def test_two_levels_without_filter_bit_exact(synth, oracle, T, W, H, nf, n, thr):
+    """Two pyramid levels on a frame whose first refined level is more than 512 cells high: the filter's descriptors
+    cannot address it, so the byte-wise k_refine<false> refines every coarse candidate unfiltered."""
+    bank = synth.synth_bank(n, num_features=nf, levels=2, seed=21, class_ids=("01_template", "02_template"))
+    q, _ = synth.synth_frame(W, H, levels=2, seed=9, bank=bank, plant=6, T=T)
+    nat, packed = _native(T, bank)
+    got = nat.match_quantized(q, thr)
+    want, st = oracle.match(q, T, packed, thr, want_stats=True)
+    assert len(want) > 0
+    _assert_same(got, want)
+    c = nat.counters()
+    assert c["coarse_candidates"] == int(st["coarse_candidates"])
+    assert c["refine_bytes"] == int(st["refine_byte_adds"])
+    assert c["filter_bytes_read"] == 0
 
 
 def test_unsafe_templates_take_the_byte_path_next_to_the_bit_sliced_one(synth, oracle):

@@ -6,7 +6,8 @@
 #   synccheck : barrier / mbarrier misuse (the TMA staging of k_coarse_packed, __syncthreads in divergent code)
 # on (a) __graft_entry__.smoke() -- one full match checked against the oracle -- and (b) the fused multi-GPU exchange
 # with three handles in one process (peer stores, ticket counters, frame flags, the collector's spin wait), and
-# (c) a second match with every alternative path switched on by environment (byte-wise refinement, 8-lane filter).
+# (c) memcheck on the matches that take the fallback kernels: byte-wise refinement without the filter, unsafe templates
+# next to eligible ones (filter + k_refine<true>, H-planes derived by k_refine_prep), three pyramid levels.
 # Usage (on a GPU box):  bash tools/sanitize.sh [outdir]      -> <outdir>/summary.txt, one log per tool x case
 set -u
 OUT=${1:-gpurun_out/sanitize}
@@ -27,6 +28,7 @@ for tool in memcheck racecheck synccheck; do
   run "$tool" smoke python -c "import __graft_entry__ as g; g.smoke()"
   run "$tool" exchange3 python -m pytest "tests/test_gpu_dist.py::test_fused_exchange_three_handles_one_process" -x -q -p no:cacheprovider
 done
-LINEMOD_B200_BITS_EXACT=0 LINEMOD_B200_FILTER_VARIANT=1 LINEMOD_B200_PLANES_DIRECT=0 run memcheck smoke_altpaths python -c "import __graft_entry__ as g; g.smoke()"
-LINEMOD_B200_FILTER=0 run memcheck smoke_nofilter python -c "import __graft_entry__ as g; g.smoke()"
+P=tests/test_gpu_match_parity.py
+run memcheck fallbacks python -m pytest -x -q -p no:cacheprovider "$P::test_two_levels_without_filter_bit_exact" \
+  "$P::test_unsafe_templates_take_the_byte_path_next_to_the_bit_sliced_one" "$P::test_match_bit_exact_synthetic[T6-640-512-96-35-70.0]"
 echo "done: $(cat "$OUT/summary.txt" | wc -l) runs" | tee -a "$OUT/summary.txt"

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Per-stage device times and counters of the match path on the bench workload (or the reference's fixture frame with the
-full allScales bank), filter on / off.  Development probe: prints one JSON line per configuration.
+full allScales bank).  Development probe: prints one JSON line.
 
   python tools/stage_probe.py [--templates 3115] [--frames 32] [--real] [--threshold 75]
 """
@@ -24,7 +24,6 @@ def main():
     ap.add_argument("--width", type=int, default=640)
     ap.add_argument("--height", type=int, default=480)
     ap.add_argument("--real", action="store_true", help="fixture frame + full allScales bank (tests/golden)")
-    ap.add_argument("--filters", default="1,0")
     args = ap.parse_args()
     lib = importlib.import_module("6dpose_b200._lib")
     synth = importlib.import_module("6dpose_b200.synth")
@@ -39,24 +38,22 @@ def main():
         packed = bank.pack(bank.class_ids(), 4)
         frames = [synth.synth_frame(args.width, args.height, levels=2, seed=1000 + i, bank=bank, plant=8, T=T)[0]
                   for i in range(min(args.frames, 16))]
-    for flt in args.filters.split(","):
-        os.environ["LINEMOD_B200_FILTER"] = flt
-        nat = lib.NativeDetector(T)
-        nat.load_bank(packed, 4)
-        for q in frames[:2]:
-            nat.match_quantized(q, args.threshold)
-        nat.set_timing(args.frames)
-        acc = {}
-        for i in range(args.frames):
-            nat.upload_quantized(frames[i % len(frames)])
-            nat.run(args.threshold)
-            for k, v in nat.counters().items():
-                acc[k] = acc.get(k, 0) + v
-        st = nat.stage_times_us()
-        nat.set_timing(0)
-        print(json.dumps({"filter": flt, "stage_us": {k: round(v, 1) for k, v in st.items()},
-                          "counters_per_frame": {k: v // args.frames for k, v in acc.items()}}))
-        nat.close()
+    nat = lib.NativeDetector(T)
+    nat.load_bank(packed, 4)
+    for q in frames[:2]:
+        nat.match_quantized(q, args.threshold)
+    nat.set_timing(args.frames)
+    acc = {}
+    for i in range(args.frames):
+        nat.upload_quantized(frames[i % len(frames)])
+        nat.run(args.threshold)
+        for k, v in nat.counters().items():
+            acc[k] = acc.get(k, 0) + v
+    st = nat.stage_times_us()
+    nat.set_timing(0)
+    print(json.dumps({"stage_us": {k: round(v, 1) for k, v in st.items()},
+                      "counters_per_frame": {k: v // args.frames for k, v in acc.items()}}))
+    nat.close()
 
 
 if __name__ == "__main__":
