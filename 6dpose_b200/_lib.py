@@ -29,6 +29,7 @@ SYMBOLS = [
     "lm_stage_times", "lm_stream", "lm_launch_count",
     "lm_set_boxes", "lm_enqueue_post", "lm_complete_post", "lm_match_top",
     "lm_peer_export", "lm_peer_base", "lm_peer_connect", "lm_peer_connect_local", "lm_peer_disconnect",
+    "lm_extract_templates",
     "lm_icp_create", "lm_icp_destroy", "lm_icp_process", "lm_icp_process_batch", "lm_icp_last_stats", "lm_icp_launch_count", "lm_icp_set_use_scene_cloud",
 ]
 
@@ -97,6 +98,7 @@ def load():
     L.lm_launch_count.restype = c_i64
     f32p, f64p = ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_double)
     u16p = ctypes.POINTER(ctypes.c_uint16)
+    L.lm_extract_templates.argtypes = [vp, c_int, c_int, u8pp, ctypes.POINTER(u16p), u8pp, c_int, c_int, i32p, i32p, i32p]
     L.lm_icp_create.argtypes = [c_int, ctypes.POINTER(vp)]
     L.lm_icp_destroy.argtypes = [vp]
     L.lm_icp_destroy.restype = None
@@ -386,6 +388,27 @@ class NativeDetector:
         check(self._L.lm_stage_times(self._h, a))
         keys = ["linear_memories", "coarse_scan", "offsets", "refine", "total", "refine_prep", "refine_filter", "refine_exact"]
         return dict(zip(keys, [float(v) for v in a]))
+
+    # ---- template extraction on the device (include/linemod_b200.h, lm_extract_templates) ----
+    def extract_templates(self, num_features, rgbs, depths, masks):
+        """Detector::addTemplate's extraction for n views of one size (uint8 HxWx3, uint16 HxW, uint8 HxW or None;
+        the caller checks dtypes and shapes).  Returns (ok bool [n], tmeta int32 [n, 2L, 4] = width, height, first,
+        count after cropTemplates, feats int32 [n, F, 3] = x, y, label with F = sum_l 2 * (num_features >> l))."""
+        n = len(rgbs)
+        rows, cols = (rgbs[0].shape[:2] if n else (0, 0))
+        F = sum(2 * (int(num_features) >> l) for l in range(self.levels))
+        ok = np.zeros(n, np.int32)
+        tmeta = np.zeros((n, 2 * self.levels, 4), np.int32)
+        feats = np.zeros((n, F, 3), np.int32)
+        u8p, u16p = ctypes.POINTER(ctypes.c_uint8), ctypes.POINTER(ctypes.c_uint16)
+        rp = (u8p * max(n, 1))(*[a.ctypes.data_as(u8p) for a in rgbs])
+        dp = (u16p * max(n, 1))(*[a.ctypes.data_as(u16p) for a in depths])
+        mp = None
+        if any(m is not None for m in masks):
+            mp = (u8p * max(n, 1))(*[m.ctypes.data_as(u8p) if m is not None else None for m in masks])
+        check(self._L.lm_extract_templates(self._h, int(num_features), n, rp, dp, mp, int(rows), int(cols), self._i32(ok),
+                                           self._i32(tmeta), self._i32(feats)))
+        return ok.astype(bool), tmeta, feats
 
     def stream(self):
         return self._L.lm_stream(self._h)

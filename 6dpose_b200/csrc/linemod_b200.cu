@@ -5,6 +5,8 @@
 //   kernels (lm_kernels.cuh): k_linear_memories_band, k_coarse_packed / k_coarse_bytes, k_scan_counts, k_refine_prep,
 //                             k_refine_filter_w, k_refine_bits / k_refine, k_peer_collect
 //   lm_finish (host)   <- std::sort + std::unique                       LL.cpp:1772-1774
+//   lm_extract_templates <- Detector::addTemplate's extraction, batched over views (lm_train.cuh; cropTemplates on
+//                           the host)                                   LL.cpp:234-318, 589-643, 888-966, 1943-1975
 // Integer results (raw scores, x, y, template ids) are bit-exact; the float similarity is produced by
 // the same two IEEE operations as the reference ((raw * 100.f) / (4 * n)).
 //
@@ -56,6 +58,9 @@ int lm_fail(int code, const char* fmt, ...) {
 #include "lm_kernels.cuh"
 #include "lm_frontend.cuh"
 #include "lm_post.cuh"
+#include "lm_train.cuh"
+
+#include <cub/device/device_segmented_sort.cuh>
 
 // Launch with programmatic stream serialization (see lm_pdl_wait in lm_kernels.cuh).
 template <typename... KArgs, typename... Args>
@@ -959,7 +964,8 @@ extern "C" int lm_upload_images(lm_detector* d, const uint8_t* rgb, const uint16
       d->launches += 1 + (masks[0] ? 1 : 0) + (masks[1] ? 1 : 0);
     }
     // colour: weak threshold 10 -> gate on squared magnitude > 100 (ColorGradient(10, nf, 55), LL.cpp:1687)
-    CU(launch_pdl(k_fe_gradient, grid2(f.cols, f.rows), dim3(FE_TW, FE_TH), 0, st, (const uint8_t*)f.src, f.rows, f.cols, 100, f.qun, f.strong));
+    CU(launch_pdl(k_fe_gradient, grid2(f.cols, f.rows), dim3(FE_TW, FE_TH), 0, st, (const uint8_t*)f.src, f.rows, f.cols, 100, f.qun, f.strong,
+                  (int32_t*)nullptr));
     CU(launch_pdl(k_fe_hysteresis, grid2(f.cols, f.rows), dim3(256), 0, st, (const uint8_t*)f.qun, (const uint8_t*)f.strong,
                   (const uint8_t*)(masks[0] ? f.mask[0] : nullptr), f.rows, f.cols, lv.d_q[0]));
     d->launches += 2;
@@ -2013,5 +2019,232 @@ extern "C" int lm_stage_times(lm_detector* d, float* out8) {
     }
   }
   for (int i = 0; i < 8; ++i) out8[i] = (float)(acc[i] / (double)n);
+  return LM_OK;
+}
+
+// ---- template extraction (Detector::addTemplate, LL.cpp:1943-1975), batched over views ---------------------------
+namespace {
+struct TrainBuffers {  // one chunk of views; freed when the call returns
+  std::vector<void*> owned;
+  ~TrainBuffers() {
+    for (void* p : owned) cudaFree(p);
+  }
+  template <typename T>
+  cudaError_t get(T** p, size_t count) {
+    *p = nullptr;
+    if (!count) return cudaSuccess;
+    cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
+    if (e == cudaSuccess) owned.push_back((void*)*p);
+    return e;
+  }
+};
+}  // namespace
+
+// cropTemplates (LL.cpp:234-277) on one view's 2L templates: common box over all levels and modalities, origin
+// rounded down to even, coordinates shifted per level; tmeta gets {width, height, first, count}.
+static void crop_view(int L, const int* first, const int* count, int32_t* feats, int32_t* tmeta) {
+  long long min_x = INT32_MAX, min_y = INT32_MAX, max_x = INT32_MIN, max_y = INT32_MIN;
+  for (int s = 0; s < 2 * L; ++s)
+    for (int i = 0; i < count[s]; ++i) {
+      const int32_t* f = feats + (size_t)(first[s] + i) * 3;
+      const long long x = (long long)f[0] << (s / 2), y = (long long)f[1] << (s / 2);
+      min_x = std::min(min_x, x); max_x = std::max(max_x, x);
+      min_y = std::min(min_y, y); max_y = std::max(max_y, y);
+    }
+  if (min_x % 2 == 1) min_x -= 1;
+  if (min_y % 2 == 1) min_y -= 1;
+  for (int s = 0; s < 2 * L; ++s) {
+    const int l = s / 2;
+    tmeta[s * 4 + 0] = (int32_t)((max_x - min_x) >> l);
+    tmeta[s * 4 + 1] = (int32_t)((max_y - min_y) >> l);
+    tmeta[s * 4 + 2] = first[s];
+    tmeta[s * 4 + 3] = count[s];
+    for (int i = 0; i < count[s]; ++i) {
+      int32_t* f = feats + (size_t)(first[s] + i) * 3;
+      f[0] -= (int32_t)(min_x >> l);
+      f[1] -= (int32_t)(min_y >> l);
+    }
+  }
+}
+
+#define LM_TRAIN_MAX_CHUNK 512
+#define LM_TRAIN_MAX_SIDE 16384
+
+extern "C" int lm_extract_templates(lm_detector* d, int num_features, int n_views, const uint8_t* const* rgb,
+                                    const uint16_t* const* depth, const uint8_t* const* masks, int rows, int cols, int32_t* ok,
+                                    int32_t* tmeta, int32_t* feats) {
+  if (!d || !rgb || !depth || !ok || !tmeta || !feats) return fail(LM_E_INVALID, "null argument");
+  if (d->device < 0) return fail(LM_E_STATE, "host-only handle (device -1): GPU stages are unavailable");
+  const int L = d->L;
+  if (n_views < 0) return fail(LM_E_INVALID, "n_views = %d", n_views);
+  if (num_features < 1 || (num_features >> (L - 1)) < 1)
+    return fail(LM_E_INVALID, "num_features = %d: every one of the %d pyramid levels needs at least one feature (num_features >> level)",
+                num_features, L);
+  if (rows < 1 || cols < 1 || rows > LM_TRAIN_MAX_SIDE || cols > LM_TRAIN_MAX_SIDE)
+    return fail(LM_E_INVALID, "image size %d x %d outside 1..%d", cols, rows, LM_TRAIN_MAX_SIDE);
+  if (rows % (1 << (L - 1)) || cols % (1 << (L - 1)))
+    return fail(LM_E_INVALID, "rows and cols must be multiples of 2^(pyramid_levels - 1) = %d for extraction on the GPU (got %d x %d)",
+                1 << (L - 1), cols, rows);
+  for (int v = 0; v < n_views; ++v)
+    if (!rgb[v] || !depth[v]) return fail(LM_E_INVALID, "null image of view %d", v);
+  if (n_views == 0) return LM_OK;
+  CU(cudaSetDevice(d->device));
+  cudaStream_t st = d->stream;
+  if (d->upper_pending) CU(cudaStreamWaitEvent(st, d->ev_upper, 0));
+  if (!d->fe_lut) {
+    uint8_t lut[400];  // as in lm_upload_images
+    for (int vy = 0; vy < 20; ++vy)
+      for (int vx = 0; vx < 20; ++vx) {
+        double a = atan2((double)(vy - 10), (double)(vx - 10)) * 180.0 / 3.14159265358979323846;
+        a = fmod(a + 360.0, 360.0);
+        lut[vy * 20 + vx] = (uint8_t)(1u << (((int)(fmod(a + 22.5, 360.0) / 45.0)) % 8));
+      }
+    CU(cudaMemcpyToSymbolAsync(c_normal_lut, lut, sizeof(lut), 0, cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));
+    d->fe_lut = true;
+  }
+
+  // layout of one view: levels l = 0..L-1 of size (rows >> l) x (cols >> l); candidate segments (level, modality)
+  // with room for every pixel of their level; features in slot order with nf >> l per slot
+  TrainSelect ts = {};
+  ts.L = L;
+  ts.nf0 = num_features;
+  int64_t key_stride = 0;
+  int key_off[LM_MAX_LEVELS];
+  int F = 0;
+  for (int l = 0; l < L; ++l) {
+    ts.cols[l] = cols >> l;
+    ts.npix[l] = (rows >> l) * (cols >> l);
+    key_off[l] = (int)key_stride;
+    key_stride += 2 * (int64_t)ts.npix[l];
+    for (int m = 0; m < 2; ++m) {
+      ts.first[l * 2 + m] = F;
+      F += num_features >> l;
+    }
+  }
+  ts.F = F;
+  const int S = 2 * L;
+  const size_t n0 = (size_t)rows * cols, n1 = L > 1 ? n0 / 4 : 0;
+  const int smem = 2 * num_features * (int)sizeof(int);
+  if (smem > 200 * 1024) return fail(LM_E_INVALID, "num_features = %d above the %d the selection kernel holds", num_features, 200 * 1024 / 8);
+  if (smem > 48 * 1024) CU(cudaFuncSetAttribute(k_tr_select, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+
+  // chunk of views resident at once: set by free device memory (half of it at most)
+  const size_t per_view = n0 * (3 + 2 + 1 + 1 + 1 + 4 + 1 + 4) + n1 * (3 + 1 + 1) + (size_t)key_stride * 16 + (size_t)F * 12 + 64 + S * 16;
+  size_t free_b = 0, total_b = 0;
+  CU(cudaMemGetInfo(&free_b, &total_b));
+  int64_t chunk = (int64_t)(free_b / 2 / per_view);
+  chunk = std::min<int64_t>(std::min<int64_t>(chunk, LM_TRAIN_MAX_CHUNK), n_views);
+  chunk = std::min<int64_t>(chunk, (int64_t)(INT32_MAX / key_stride));
+  if (chunk < 1) return fail(LM_E_CUDA, "not enough free device memory for one view (%zu bytes)", per_view);
+  const int B = (int)chunk;
+
+  TrainBuffers tb;
+  uint8_t *rgbA, *rgbB, *maskA, *maskB, *normA, *normB, *angle, *nfg, *qun, *strong, *nraw, *nq, *has_mask, *seg_fail;
+  uint16_t* dep;
+  int32_t *mag, *g, *d_feats, *seg_begin, *seg_end, *lcount, *area;
+  unsigned long long *keys, *keys_sorted;
+  CU(tb.get(&rgbA, B * n0 * 3)); CU(tb.get(&rgbB, B * n1 * 3)); CU(tb.get(&dep, B * n0));
+  CU(tb.get(&maskA, B * n0)); CU(tb.get(&maskB, B * n1)); CU(tb.get(&normA, B * n0)); CU(tb.get(&normB, B * n1));
+  CU(tb.get(&angle, B * n0)); CU(tb.get(&mag, B * n0)); CU(tb.get(&nfg, B * n0)); CU(tb.get(&g, B * n0));
+  CU(tb.get(&qun, n0)); CU(tb.get(&strong, n0)); CU(tb.get(&nraw, n0)); CU(tb.get(&nq, n0));
+  CU(tb.get(&has_mask, (size_t)B)); CU(tb.get(&seg_fail, (size_t)B * S));
+  CU(tb.get(&seg_begin, (size_t)B * S)); CU(tb.get(&seg_end, (size_t)B * S));
+  CU(tb.get(&lcount, (size_t)B * L * 8)); CU(tb.get(&area, (size_t)B * L));
+  CU(tb.get(&keys, (size_t)B * key_stride)); CU(tb.get(&keys_sorted, (size_t)B * key_stride));
+  CU(tb.get(&d_feats, (size_t)B * F * 3));
+  std::vector<int32_t> h_begin((size_t)B * S);
+  for (int v = 0; v < B; ++v)
+    for (int l = 0; l < L; ++l)
+      for (int m = 0; m < 2; ++m) h_begin[(size_t)v * S + l * 2 + m] = (int32_t)(v * key_stride + key_off[l] + m * (int64_t)ts.npix[l]);
+  CU(cudaMemcpyAsync(seg_begin, h_begin.data(), h_begin.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  size_t sort_bytes = 0;
+  CU(cub::DeviceSegmentedSort::SortKeys(nullptr, sort_bytes, keys, keys_sorted, (int)(B * key_stride), B * S, seg_begin, seg_end, st));
+  void* sort_tmp = nullptr;
+  CU(tb.get((uint8_t**)&sort_tmp, sort_bytes));
+  std::vector<uint8_t> h_has(B), h_fail((size_t)B * S);
+
+  auto grid2 = [](int w, int h, int z) { return dim3((unsigned)((w + 31) / 32), (unsigned)((h + 7) / 8), (unsigned)z); };
+  for (int v0 = 0; v0 < n_views; v0 += B) {
+    const int nb = std::min(B, n_views - v0);
+    for (int v = 0; v < nb; ++v) {
+      const uint8_t* mk = masks ? masks[v0 + v] : nullptr;
+      h_has[v] = mk != nullptr;
+      CU(cudaMemcpyAsync(rgbA + v * n0 * 3, rgb[v0 + v], n0 * 3, cudaMemcpyHostToDevice, st));
+      CU(cudaMemcpyAsync(dep + v * n0, depth[v0 + v], n0 * 2, cudaMemcpyHostToDevice, st));
+      if (mk) CU(cudaMemcpyAsync(maskA + v * n0, mk, n0, cudaMemcpyHostToDevice, st));
+    }
+    CU(cudaMemcpyAsync(has_mask, h_has.data(), nb, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(seg_end, seg_begin, (size_t)nb * S * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    CU(cudaMemsetAsync(lcount, 0, (size_t)nb * L * 8 * sizeof(int32_t), st));
+    CU(cudaMemsetAsync(area, 0, (size_t)nb * L * sizeof(int32_t), st));
+    for (int l = 0; l < L; ++l) {
+      const int H = rows >> l, W = cols >> l;
+      // level l lives in the A buffers for even l and in the B buffers for odd l (per-view strides n0 / n1)
+      uint8_t* rgb_l = (l & 1) ? rgbB : rgbA;
+      uint8_t* norm_l = (l & 1) ? normB : normA;
+      uint8_t* mask_l = (l & 1) ? maskB : maskA;
+      const size_t s_l = (l & 1) ? n1 : n0;
+      const size_t s_u = (l & 1) ? n0 : n1;  // stride of level l - 1
+      for (int v = 0; v < nb; ++v) {
+        if (l > 0) {  // ColorGradientPyramid::pyrDown / DepthNormalPyramid::pyrDown (LL.cpp:557-567, 861-879)
+          const uint8_t* rgb_u = ((l & 1) ? rgbA : rgbB) + v * s_u * 3;
+          const uint8_t* norm_u = ((l & 1) ? normA : normB) + v * s_u;
+          CU(launch_pdl(k_fe_pyrdown, grid2(W, H, 1), dim3(256), 0, st, rgb_u, H * 2, W * 2, rgb_l + v * s_l * 3, H, W));
+          CU(launch_pdl(k_fe_decimate, grid2(W, H, 1), dim3(256), 0, st, norm_u, W * 2, norm_l + v * s_l, H, W, (const uint8_t*)nullptr,
+                        (uint8_t*)nullptr));
+          d->launches += 2;
+          if (h_has[v]) {
+            const uint8_t* mask_u = ((l & 1) ? maskA : maskB) + v * s_u;
+            CU(launch_pdl(k_fe_decimate, grid2(W, H, 1), dim3(256), 0, st, mask_u, W * 2, mask_l + v * s_l, H, W, (const uint8_t*)nullptr,
+                          (uint8_t*)nullptr));
+            ++d->launches;
+          }
+        }
+        // colour labels WITHOUT the mask (pyr.angle) and the squared magnitude
+        CU(launch_pdl(k_fe_gradient, grid2(W, H, 1), dim3(FE_TW, FE_TH), 0, st, (const uint8_t*)(rgb_l + v * s_l * 3), H, W, 100, qun, strong,
+                      mag + v * n0));
+        CU(launch_pdl(k_fe_hysteresis, grid2(W, H, 1), dim3(256), 0, st, (const uint8_t*)qun, (const uint8_t*)strong, (const uint8_t*)nullptr,
+                      H, W, angle + v * n0));
+        d->launches += 2;
+        if (l == 0) {
+          CU(launch_pdl(k_fe_normals, grid2(W, H, 1), dim3(256), 0, st, (const uint16_t*)(dep + v * n0), H, W, 2000, 50, nraw));
+          CU(launch_pdl(k_fe_median, grid2(W, H, 1), dim3(256), 0, st, (const uint8_t*)nraw, (const uint8_t*)nullptr, H, W, norm_l + v * n0, nq));
+          d->launches += 2;
+        }
+      }
+      CU(launch_pdl(k_tr_prep, grid2(W, H, nb), dim3(256), 0, st, H, W, l, L, (const uint8_t*)angle, (const int32_t*)mag, n0,
+                    (const uint8_t*)norm_l, (const uint8_t*)mask_l, s_l, (const uint8_t*)has_mask, keys, seg_end, nfg, area));
+      CU(launch_pdl(k_tr_coldist, dim3((unsigned)((W + 127) / 128), 1, (unsigned)nb), dim3(128), 0, st, H, W, (const uint8_t*)nfg, n0, g));
+      CU(launch_pdl(k_tr_normcand, grid2(W, H, nb), dim3(256), 0, st, H, W, l, L, 2 >> l, (const uint8_t*)nfg, (const int*)g, n0, keys,
+                    seg_end, lcount));
+      d->launches += 3;
+    }
+    CU(launch_pdl(k_tr_normscore, dim3(16, (unsigned)(nb * L)), dim3(256), 0, st, keys, (const int*)seg_begin, (const int*)seg_end,
+                  (const int*)lcount));
+    ++d->launches;
+    CU(cub::DeviceSegmentedSort::SortKeys(sort_tmp, sort_bytes, keys, keys_sorted, (int)(nb * key_stride), nb * S, seg_begin, seg_end, st));
+    CU(launch_pdl(k_tr_select, dim3((unsigned)(nb * S)), dim3(32), (size_t)smem, st, ts, (const unsigned long long*)keys_sorted,
+                  (const int*)seg_begin, (const int*)seg_end, (const uint8_t*)has_mask, (const int*)area, d_feats, seg_fail));
+    ++d->launches;
+    CU(cudaMemcpyAsync(feats + (size_t)v0 * F * 3, d_feats, (size_t)nb * F * 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_fail.data(), seg_fail, (size_t)nb * S, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    CU(cudaGetLastError());
+    int count[2 * LM_MAX_LEVELS];
+    for (int s = 0; s < S; ++s) count[s] = num_features >> (s / 2);
+    for (int v = 0; v < nb; ++v) {
+      bool good = true;
+      for (int s = 0; s < S; ++s) good = good && !h_fail[(size_t)v * S + s];
+      ok[v0 + v] = good ? 1 : 0;
+      int32_t* tm = tmeta + (size_t)(v0 + v) * S * 4;
+      int32_t* fv = feats + (size_t)(v0 + v) * F * 3;
+      if (good) crop_view(L, ts.first, count, fv, tm);
+      else {
+        memset(tm, 0, (size_t)S * 4 * sizeof(int32_t));
+        memset(fv, 0, (size_t)F * 3 * sizeof(int32_t));
+      }
+    }
+  }
   return LM_OK;
 }

@@ -47,9 +47,11 @@ __device__ __forceinline__ int fe_phase_bin(float x, float y) {
   return __float2int_rn(__fmul_rn(a, 0.044444445f));  // 16/360 as float, round half to even
 }
 
-// src u8 [H][W][3]; out: qun u8 [H][W] = (bin & 7) in the interior, 0 on the border; strong u8 = mag > thr_sq
+// src u8 [H][W][3]; out: qun u8 [H][W] = (bin & 7) in the interior, 0 on the border; strong u8 = mag > thr_sq;
+// mag (nullable, template extraction only): the squared magnitude of the picked channel, an exact integer <= 2 * 1020^2
 __global__ void __launch_bounds__(FE_TW * FE_TH) k_fe_gradient(const uint8_t* __restrict__ src, int H, int W, int thr_sq,
-                                                              uint8_t* __restrict__ qun, uint8_t* __restrict__ strong) {
+                                                              uint8_t* __restrict__ qun, uint8_t* __restrict__ strong,
+                                                              int32_t* __restrict__ mag) {
   lm_pdl_wait();
   __shared__ uint8_t s_in[FE_TH + 8][FE_TW + 8][3];
   __shared__ uint16_t s_h[FE_TH + 8][FE_TW + 2][3];
@@ -123,6 +125,7 @@ __global__ void __launch_bounds__(FE_TW * FE_TH) k_fe_gradient(const uint8_t* __
   if (!(x == 0 || y == 0 || x == W - 1 || y == H - 1)) bin = fe_phase_bin((float)bdx, (float)bdy) & 7;
   qun[(size_t)y * W + x] = (uint8_t)bin;
   strong[(size_t)y * W + x] = bm > thr_sq ? 1 : 0;
+  if (mag) mag[(size_t)y * W + x] = bm;
 }
 
 // 3x3 vote among the 8 bins, gate on the magnitude, >= 5 votes, optional mask (LL.cpp:457-505, 583-587)

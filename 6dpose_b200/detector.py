@@ -2,8 +2,8 @@
 
 `Detector`, `Match` and `poseRefine` keep the reference's names, argument order, keyword names and
 error behaviour; underneath, `Detector.match` calls the C-ABI library (CUDA, sm_100a) through
-ctypes.  The quantization front-end (cv2) and template extraction run on the host, as SURVEY.md
-section 8 rows a14 / f2 describe.
+ctypes.  The quantization front-end runs on the GPU (or cv2, `Detector.frontend`); addTemplate extracts on the
+host (cv2, as the reference does) and addTemplates extracts many views at once on the GPU.
 """
 import os
 
@@ -99,6 +99,21 @@ class Detector:
         if tid >= 0:
             self._bank_dirty = True
         return tid
+
+    def addTemplates(self, sources_list, class_id, object_masks):
+        """Beyond the reference: addTemplate for many views of one size, extracted on the GPU in one call
+        (lm_extract_templates).  Returns list[int] of template ids (-1 where extraction fails), and leaves the bank,
+        feature for feature, as [addTemplate(s, class_id, m) for s, m in zip(sources_list, object_masks)] would.
+        object_masks entries may be None or empty (no mask).  The image size must be a multiple of
+        2^(pyramid_levels - 1); addTemplate serves other sizes."""
+        from . import training
+        if self._native is None:
+            self._native = _lib.NativeDetector(self.T_at_level, self.device)
+            self._bank_dirty = True
+        ids = training.add_templates(self, self._native, list(sources_list), class_id, list(object_masks))
+        if any(i >= 0 for i in ids):
+            self._bank_dirty = True
+        return ids
 
     def getTemplates(self, class_id, template_id):
         # The reference returns std::vector<Template>, a type pybind11.cpp never registers: calling it

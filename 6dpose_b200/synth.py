@@ -157,3 +157,22 @@ def synth_rgbd(W=640, H=480, seed=7):
     depth[rng.random((H, W)) < 0.03] = 0   # sensor holes
     depth[:, : W // 10] = 2600              # beyond the distance threshold
     return rgb, np.clip(depth, 0, 65535).astype(np.uint16)
+
+
+def warp_views(rgb, depth, mask, n, seed=0, max_angle=30.0, scale=(0.8, 1.2), max_shift=40):
+    """n training views from one (rgb, depth, mask) view under seeded in-plane rotation, scale and shift about the
+    mask's centre: rgb interpolated linearly, depth and mask nearest (no renderer is needed to grow a bank for
+    extraction tests and timings).  Returns a list of (rgb, depth, mask)."""
+    import cv2
+    rng = np.random.default_rng(seed)
+    H, W = depth.shape
+    ys, xs = np.nonzero(mask)
+    cx, cy = (float(xs.mean()), float(ys.mean())) if xs.size else (W / 2.0, H / 2.0)
+    out = []
+    for _ in range(n):
+        M = cv2.getRotationMatrix2D((cx, cy), float(rng.uniform(-max_angle, max_angle)), float(rng.uniform(*scale)))
+        M[:, 2] += rng.uniform(-max_shift, max_shift, 2)
+        out.append((cv2.warpAffine(rgb, M, (W, H), flags=cv2.INTER_LINEAR),
+                    cv2.warpAffine(depth, M, (W, H), flags=cv2.INTER_NEAREST),
+                    cv2.warpAffine(mask, M, (W, H), flags=cv2.INTER_NEAREST)))
+    return out

@@ -10,6 +10,9 @@ linemodLevelup/linemodLevelup.cpp, "LL.cpp"):
   extract_normal_template     <- DepthNormalPyramid::extractTemplate        LL.cpp:888-966
   crop_templates              <- cropTemplates                              LL.cpp:234-277
   add_template                <- Detector::addTemplate                      LL.cpp:1943-1975
+
+add_templates is the batched GPU path (lm_extract_templates, csrc/lm_train.cuh): the same templates, feature for
+feature, for many views in one call.
 """
 import math
 
@@ -146,22 +149,41 @@ def crop_templates(templates):
     return min_x, min_y, max_x - min_x, max_y - min_y
 
 
+def _check_mask(object_mask):
+    if object_mask is None or not np.asarray(object_mask).size:
+        return None
+    mask = np.ascontiguousarray(object_mask)
+    if mask.ndim == 3:
+        raise TypeError("object_mask must be single channel")
+    if mask.dtype != np.uint8:
+        raise TypeError("object_mask must be uint8 (255 = object)")
+    return mask
+
+
+def class_templates(detector, class_id):
+    """class_templates[class_id] (LL.cpp:1947): created even when every extraction fails.  A class loaded from a
+    packed bank file is unpacked to a list before it grows."""
+    pyramids = detector.bank.classes.setdefault(class_id, [])
+    if not isinstance(pyramids, list):
+        pyramids = detector.bank.classes[class_id] = list(pyramids)
+    return pyramids
+
+
+def append_template(pyramids, tp, cropped=False):
+    """The end of Detector::addTemplate (LL.cpp:1962-1974): cropTemplates, then the pyramid gets the next id."""
+    if not cropped:
+        crop_templates(tp)
+    pyramids.append(tp)
+    return len(pyramids) - 1
+
+
 def add_template(detector, sources, class_id, object_mask):
     """Detector::addTemplate (LL.cpp:1943-1975): template id, or -1 when extraction fails."""
     if len(sources) != 2:
         raise RuntimeError("sources.size() == modalities.size()")
     src = [detector._as_source(s, i) for i, s in enumerate(sources)]
-    mask = None
-    if object_mask is not None and np.asarray(object_mask).size:
-        mask = np.ascontiguousarray(object_mask)
-        if mask.ndim == 3:
-            raise TypeError("object_mask must be single channel")
-        if mask.dtype != np.uint8:
-            raise TypeError("object_mask must be uint8 (255 = object)")
-    pyramids = detector.bank.classes.setdefault(class_id, [])  # class_templates[class_id], even on failure
-    if not isinstance(pyramids, list):  # loaded from a packed bank file: unpack before growing it
-        pyramids = detector.bank.classes[class_id] = list(pyramids)
-    template_id = len(pyramids)
+    mask = _check_mask(object_mask)
+    pyramids = class_templates(detector, class_id)
     L = detector.pyramid_levels
     nf = detector.num_features
     tp = [None] * (2 * L)
@@ -177,6 +199,39 @@ def add_template(detector, sources, class_id, object_mask):
             if t is None:
                 return -1
             tp[l * 2 + m] = t
-    crop_templates(tp)
-    pyramids.append(tp)
-    return template_id
+    return append_template(pyramids, tp)
+
+
+def add_templates(detector, native, sources_list, class_id, object_masks):
+    """add_template over many views of one size, extracted on the GPU in one call (lm_extract_templates; cropTemplates
+    runs inside the library).  Same ids and bank as calling add_template per view in order.  Every input is checked
+    before the bank changes: a bad view raises and adds nothing."""
+    if len(object_masks) != len(sources_list):
+        raise RuntimeError("%d object masks for %d views" % (len(object_masks), len(sources_list)))
+    rgbs, deps, masks = [], [], []
+    for sources, object_mask in zip(sources_list, object_masks):
+        if len(sources) != 2:
+            raise RuntimeError("sources.size() == modalities.size()")
+        rgb, dep = detector._as_source(sources[0], 0), detector._as_source(sources[1], 1)
+        mask = _check_mask(object_mask)
+        shape = rgbs[0].shape[:2] if rgbs else rgb.shape[:2]
+        if rgb.shape[:2] != shape or dep.shape != shape:
+            raise RuntimeError("all views of one addTemplates call must have one size: %r, then rgb %r / depth %r"
+                               % (shape, rgb.shape[:2], dep.shape))
+        if mask is not None and mask.shape != shape:
+            raise RuntimeError("mask.size() == source.size(): mask %r for images %r" % (mask.shape, shape))
+        rgbs.append(rgb)
+        deps.append(dep)
+        masks.append(mask)
+    if not rgbs:
+        return []
+    ok, tmeta, feats = native.extract_templates(detector.num_features, rgbs, deps, masks)
+    pyramids = class_templates(detector, class_id)
+    ids = []
+    for v in range(len(rgbs)):
+        if not ok[v]:
+            ids.append(-1)
+            continue
+        tp = [Template(w, h, s_ // 2, feats[v, b:b + n].copy()) for s_, (w, h, b, n) in enumerate(tmeta[v].tolist())]
+        ids.append(append_template(pyramids, tp, cropped=True))
+    return ids

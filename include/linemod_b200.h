@@ -193,6 +193,26 @@ int lm_match_quantized(lm_detector* d, const uint8_t* const* quantized, const in
 int lm_match_images(lm_detector* d, const uint8_t* rgb, const uint16_t* depth, int rows, int cols, const uint8_t* mask_color,
                     const uint8_t* mask_depth, float threshold, lm_match* out, int64_t cap, int64_t* n_out);
 
+/* Template extraction of Detector::addTemplate (LL.cpp:1943-1975) for n_views views at once, on this handle's
+ * device and stream with its pyramid levels L; the loaded bank and the uploaded frame are not touched.  View v is
+ * rgb[v] (u8 rows x cols x 3), depth[v] (u16 rows x cols, mm) and masks[v] (u8 rows x cols, nonzero = object; masks
+ * NULL or masks[v] NULL = no mask).  Per view and pyramid level it runs the GPU front-end of lm_upload_images
+ * (labels without the mask), then ColorGradientPyramid::extractTemplate (LL.cpp:589-643: mask border, squared
+ * magnitude > 55^2) and DepthNormalPyramid::extractTemplate (LL.cpp:888-966: mask eroded twice, per-label
+ * chessboard distance transform, score = distance / candidates of the label), the stable sort by score and
+ * selectScatteredFeatures (LL.cpp:279-318) with the reference's float32 arithmetic, and cropTemplates
+ * (LL.cpp:234-277) on the host.  Outputs, feature for feature what the reference produces:
+ *   ok[n_views]                  1 = extracted, 0 = too few candidates for some level / modality (addTemplate -1)
+ *   tmeta[n_views][2L][4]        {width, height, first, count} per slot level*2 + modality, cropped; count =
+ *                                num_features >> level, first = offset of the slot inside the view's features
+ *   feats[n_views][F][3]         {x, y, label} in selection order, F = sum over levels of 2 * (num_features >> level)
+ * Entries of views with ok = 0 are zero.  Views go through in chunks sized by free device memory.  LM_E_INVALID: a
+ * null pointer, num_features >> (L - 1) < 1, rows or cols not a multiple of 2^(L-1) (the GPU pyrDown and
+ * decimation serve even sizes; the host addTemplate serves the others) or above 16384.  A host-only handle
+ * (device -1) gets LM_E_STATE.  Blocking. */
+int lm_extract_templates(lm_detector* d, int num_features, int n_views, const uint8_t* const* rgb, const uint16_t* const* depth,
+                         const uint8_t* const* masks, int rows, int cols, int32_t* ok, int32_t* tmeta, int32_t* feats);
+
 /* ---- introspection used by the parity tests and the benchmark ---- */
 /* Quantized label image of (level, modality) of the uploaded frame: rows*cols bytes. */
 int lm_debug_quantized(lm_detector* d, int level, int modality, uint8_t* out, int64_t cap);

@@ -7,7 +7,8 @@
 # on (a) __graft_entry__.smoke() -- one full match checked against the oracle -- and (b) the fused multi-GPU exchange
 # with three handles in one process (peer stores, ticket counters, frame flags, the collector's spin wait), and
 # (c) memcheck on the matches that take the fallback kernels: byte-wise refinement without the filter, unsafe templates
-# next to eligible ones (filter + k_refine<true>, H-planes derived by k_refine_prep), three pyramid levels.
+# next to eligible ones (filter + k_refine<true>, H-planes derived by k_refine_prep), three pyramid levels, and
+# (d) memcheck on template extraction (lm_extract_templates: tests/test_gpu_training.py).
 # Usage (on a GPU box):  bash tools/sanitize.sh [outdir]      -> <outdir>/summary.txt, one log per tool x case
 set -u
 OUT=${1:-gpurun_out/sanitize}
@@ -31,4 +32,5 @@ done
 P=tests/test_gpu_match_parity.py
 run memcheck fallbacks python -m pytest -x -q -p no:cacheprovider "$P::test_two_levels_without_filter_bit_exact" \
   "$P::test_unsafe_templates_take_the_byte_path_next_to_the_bit_sliced_one" "$P::test_match_bit_exact_synthetic[T6-640-512-96-35-70.0]"
+run memcheck training python -m pytest -x -q -p no:cacheprovider tests/test_gpu_training.py
 echo "done: $(cat "$OUT/summary.txt" | wc -l) runs" | tee -a "$OUT/summary.txt"
